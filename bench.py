@@ -2,7 +2,7 @@
 """bench.py — headline benchmark: local_laplacian (8 levels, alpha=1, beta=1) on synthetic uint16
 frames, Mpixels/s (1 Mpx = 1e6 output pixels W*H, channels not counted).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Default workload = the north-star configuration of BASELINE.json: ONE 16384x16384x3 uint16 frame, levels=8,
 alpha=1/7 (the harness passes alpha/(levels-1), apps/local_laplacian/process.cpp:31), beta=1.  At N=1 the whole
@@ -14,6 +14,9 @@ input rows from its neighbours and gathers one coarse pyramid level (halide_b200
 One JSON line on stdout (rank 0).  `value` is device-resident throughput (inputs in HBM), timed with CUDA events on
 the launch stream over exactly K steps, max over ranks; `e2e` is the same metric through the C ABI with HOST
 (pinned) buffers, H2D + D2H inside the timed region, one caller thread (the same form at every N).
+`--dump-outputs DIR` writes what the last timed step returned to DIR/output.npy (DIR/output_rank<r>.npy per rank when
+sharded) as float32: the whole output frame when it is small enough, else a fixed seeded sample of its elements.  The
+inputs are seeded too, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times the CPU oracle (a port of the reference's algorithm — libHalide needs LLVM and cannot be
 built in this image) on the box's host cores for the same config, on a bounded sample of the frame.
 """
@@ -33,6 +36,7 @@ LEVELS = 8
 ALPHA = 1.0 / 7.0   # alpha=1 divided by (levels-1), as process.cpp:31 does
 BETA = 1.0
 BYTES_PER_PX = 12   # SURVEY.md §8(d): 3 ch x 2 B in + 3 ch x 2 B out
+DUMP_ELEMENTS = 15 << 20   # float32 values --dump-outputs writes over all ranks: 60 MB, within a 64 MB budget
 
 WORKLOADS = {
     # name: (W, H) of the whole frame
@@ -187,6 +191,21 @@ def cpu_oracle_rate(W, H, budget_s=12.0, max_steps=8):
             "ms": best * 1e3, "published_reference": PUBLISHED_HALIDE_CPU}
 
 
+def dump_outputs(directory, out, rank, world):
+    """Saves one rank's output frame (uint16 on the device) as float32: whole when it fits this rank's share of
+    DUMP_ELEMENTS, else the elements at a fixed seeded set of flat positions (the same set for the same shape)."""
+    import numpy as np
+    import torch
+    flat = out.view(torch.int16).reshape(-1)   # (uint16 tensors support few ops; int16 carries the same bits)
+    limit = DUMP_ELEMENTS // world
+    if flat.numel() > limit:
+        idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), limit))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    values = flat.cpu().numpy().view(np.uint16).astype(np.float32)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "output.npy" if world == 1 else f"output_rank{rank}.npy"), values)
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU algorithm (oracle port) on the host cores."""
     if rank != 0:
@@ -202,8 +221,11 @@ def run_reference(args, rank, world):
         pyoracle.local_laplacian(img, LEVELS, ALPHA, BETA)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        pyoracle.local_laplacian(img, LEVELS, ALPHA, BETA)
+        out = pyoracle.local_laplacian(img, LEVELS, ALPHA, BETA)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        import torch
+        dump_outputs(args.dump_outputs, torch.from_numpy(out.view(np.int16)), 0, 1)
     val = W * rows / 1e6 / dt
     sample = f"{args.steps} steps of a {W}x{rows}x3 band ({'full frame' if rows == H else 'the top rows of the frame'})"
     line = {"impl": "reference", "metric": "local_laplacian Mpixels/s", "value": val, "unit": "Mpixels/s",
@@ -293,6 +315,8 @@ def run_ours(args, rank, world, local_rank):
     sampler.stop()
     launches = halide_b200.capi.halide_b200_kernel_launch_count() - n0
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs:   # (before anything below reuses the output buffers)
+        dump_outputs(args.dump_outputs, outs[(args.steps - 1) % NSETS], rank, world)
     if dist is not None:
         tt = torch.tensor([ms_total], device=dev)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -468,7 +492,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":

@@ -116,10 +116,6 @@ def set_threads(n):
     lib().oracle_set_num_threads(int(n))
 
 
-def ref_blur_available():
-    return os.path.exists(_REF_BLUR)
-
-
 def ref_blur(inp, fast=False):
     """The REFERENCE's own C blur (apps/blur/test.cpp:18-33 / :35-132) via oracle/_ref.
     inp: uint16 [h, w] -> uint16 [h-2, w-8] (the shapes test.cpp uses)."""

@@ -13,7 +13,9 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-from test_image_io import FORMAT_CASES, NAMES, REF, TNAME, random_image, samples, write_dump  # noqa: E402
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+from make_reference_golden import REF_IO as REF, write_dump  # noqa: E402
+from test_image_io import FORMAT_CASES, NAMES, TNAME, random_image, samples  # noqa: E402
 
 
 def main():

@@ -2,7 +2,7 @@
 import numpy as np
 import pytest
 
-from util import run_blur, u16_frame
+from util import reference, run_blur, sha, u16_frame
 
 pytestmark = pytest.mark.gpu
 
@@ -15,15 +15,14 @@ def test_blur_matches_oracle(hb, oracle, h, w, seed):
     assert np.array_equal(got, oracle.blur(inp))
 
 
-def test_blur_matches_reference_c_on_harness_shape(hb, oracle):
+def test_blur_matches_reference_c_on_harness_shape(hb):
     """apps/blur/test.cpp:162-191: 2568x1922 input, rand() & 0xfff, compared on the interior
-    against the reference's own C implementations (oracle/_ref)."""
-    if not oracle.ref_blur_available():
-        pytest.skip("oracle/_ref/libref_blur.so not present")
+    against the reference's own C implementations (its naive and its SSE blur)."""
     inp = u16_frame((1922, 2568), 7, bits=12)
     got = run_blur(hb, inp, (1920, 2560))
-    assert np.array_equal(got, oracle.ref_blur(inp, fast=False))
-    assert np.array_equal(got, oracle.ref_blur(inp, fast=True))
+    want = reference()["blur"]["1922x2568"]
+    assert sha(got) == want["slow"]
+    assert sha(got) == want["fast"]
 
 
 def test_blur_config1_1080p(hb, oracle):

@@ -1,24 +1,32 @@
-"""halide_b200/image_io.py against the reference's own image I/O header (tools/halide_image_io.h), which is compiled in
-place into oracle/_ref/ref_image_io (oracle/ref_image_io_tool.cpp): element conversions for every type pair, every
-format both ways (the reference writes / we read, we write / the reference reads), and the type / dimensionality choice
-of convert_and_save_image.  Where the reference binary is not available (a box without /root/reference and without
-a prebuilt oracle/_ref), the committed golden vectors (tests/golden/image_io_golden.npz, made by
-tests/golden/make_image_io_golden.py with the same binary) stand in for it."""
+"""halide_b200/image_io.py against the reference's own image I/O header (tools/halide_image_io.h): element conversions
+for every type pair, every format both ways, and the type / dimensionality choice of convert_and_save_image.  What the
+reference computed on these inputs is committed under tests/golden/: the vectors of image_io_golden.npz
+(tests/golden/make_image_io_golden.py), and digests of its whole outputs plus its sample images, cut short
+(reference_digests.json and images/, tests/golden/make_reference_golden.py).  Both scripts ran the header compiled in
+place (oracle/ref_image_io_tool.cpp)."""
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 from halide_b200 import image_io
+from util import reference, sha
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "ref_image_io")
 GOLDEN = os.path.join(ROOT, "tests", "golden", "image_io_golden.npz")
+IMAGES = os.path.join(ROOT, "tests", "golden", "images")
 NAMES = {"u8": np.uint8, "u16": np.uint16, "u32": np.uint32, "u64": np.uint64, "i8": np.int8, "i16": np.int16,
          "i32": np.int32, "i64": np.int64, "f32": np.float32, "f64": np.float64}
 TNAME = {np.dtype(v): k for k, v in NAMES.items()}
-have_ref = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/ref_image_io not built")
+
+
+def file_sha(path):
+    with open(path, "rb") as f:
+        return sha(f.read())
+
+
+def case_id(fmt, dtype, shape):
+    return f"{fmt}-{TNAME[np.dtype(dtype)]}-{'x'.join(map(str, shape))}"
 
 
 def samples(dtype, n=2048, seed=0):
@@ -37,36 +45,13 @@ def samples(dtype, n=2048, seed=0):
     return np.concatenate([edge, rng.random(n).astype(dt), (rng.random(64) * 8 - 4).astype(dt)])
 
 
-def ref_convert(a, dst, tmp_path):
-    src_f, dst_f = str(tmp_path / "in.bin"), str(tmp_path / "out.bin")
-    a.tofile(src_f)
-    subprocess.run([REF, "convert", TNAME[a.dtype], dst, src_f, dst_f], check=True)
-    return np.fromfile(dst_f, dtype=NAMES[dst])
-
-
-def write_dump(a, path):
-    with open(path, "wb") as f:
-        f.write((" ".join([TNAME[a.dtype], str(a.ndim)] + [str(e) for e in reversed(a.shape)]) + "\n").encode())
-        f.write(np.ascontiguousarray(a).tobytes())
-
-
-def read_dump(path):
-    b = open(path, "rb").read()
-    nl = b.index(b"\n")
-    parts = b[:nl].decode().split()
-    ext = [int(e) for e in parts[2:2 + int(parts[1])]]
-    return np.frombuffer(b[nl + 1:], dtype=NAMES[parts[0]]).reshape(tuple(reversed(ext))).copy()
-
-
-@have_ref
 @pytest.mark.parametrize("src", list(NAMES))
-def test_convert_matches_reference_for_every_target(src, tmp_path):
+def test_convert_matches_reference_for_every_target(src):
     a = samples(NAMES[src], seed=len(src))
     for dst in NAMES:
-        want = ref_convert(a, dst, tmp_path)
         got = image_io.convert(a, NAMES[dst])
-        assert got.dtype == want.dtype
-        assert np.array_equal(got.view(np.uint8), want.view(np.uint8)), (src, dst, a[np.flatnonzero(got != want)[:4]])
+        assert got.dtype == np.dtype(NAMES[dst]) and got.shape == a.shape
+        assert sha(got) == reference()["convert"][src][dst], (src, dst)
 
 
 def test_convert_matches_golden_vectors():
@@ -108,59 +93,43 @@ def random_image(dtype, shape, seed):
     return rng.integers(info.min, info.max, shape, dtype=dt, endpoint=True)
 
 
-@have_ref
 @pytest.mark.parametrize("fmt,dtype,shape", FORMAT_CASES)
 def test_formats_round_trip_through_the_reference(fmt, dtype, shape, tmp_path):
+    """Our writer produces the reference's bytes (a .mat file carries its own file name as the variable name, hence the
+    reference's name img.<fmt>), and our reader decodes them to the array written (the reference read its own file back
+    to the same array when the digest was made)."""
     a = random_image(dtype, shape, len(shape) * 7 + np.dtype(dtype).itemsize)
-    (tmp_path / "r").mkdir()
-    (tmp_path / "o").mkdir()
-    # (same base name in two directories: a .mat file carries its own file name as the variable name)
-    dump, ref_file, our_file, back = (str(tmp_path / n) for n in ("a.dump", "r/img." + fmt, "o/img." + fmt, "b.dump"))
-    # the reference writes, we read
-    write_dump(a, dump)
-    subprocess.run([REF, "save", dump, ref_file], check=True)
-    got = image_io.load(ref_file)
-    assert got.dtype == a.dtype and np.array_equal(got, a)
-    # we write, the reference reads
+    our_file = str(tmp_path / ("img." + fmt))
     image_io.save(a, our_file)
-    subprocess.run([REF, "load", our_file, back], check=True)
-    assert np.array_equal(read_dump(back), a)
-    if fmt in ("pgm", "ppm", "npy", "tmp", "mat"):   # these writers are byte-for-byte the reference's
-        assert open(our_file, "rb").read() == open(ref_file, "rb").read()
+    assert file_sha(our_file) == reference()["formats"][case_id(fmt, dtype, shape)]
+    got = image_io.load(our_file)
+    assert got.dtype == a.dtype and np.array_equal(got, a)
 
 
-@have_ref
-@pytest.mark.parametrize("fmt", ["pgm", "ppm", "npy", "tmp", "mat"])
+AUTOSAVE_SHAPES = {"pgm": [(6, 7)], "ppm": [(3, 6, 7)], "npy": [(5,), (6, 7), (3, 6, 7)], "tmp": [(6, 7), (3, 6, 7), (2, 3, 6, 7)],
+                   "mat": [(6, 7), (3, 6, 7)]}
+
+
+@pytest.mark.parametrize("fmt", list(AUTOSAVE_SHAPES))
 def test_convert_and_save_picks_the_reference_type(fmt, tmp_path):
-    shapes = {"pgm": [(6, 7)], "ppm": [(3, 6, 7)], "npy": [(5,), (6, 7), (3, 6, 7)], "tmp": [(6, 7), (3, 6, 7), (2, 3, 6, 7)],
-              "mat": [(6, 7), (3, 6, 7)]}[fmt]
-    for shape in shapes:
+    """convert_and_save_image writes the reference's file byte for byte: the same element type and dimensionality
+    chosen for the format, the same converted values."""
+    for shape in AUTOSAVE_SHAPES[fmt]:
         for src in NAMES.values():
-            a = random_image(src, shape, 3)
-            dump, ref_file, our_file, d1, d2 = (str(tmp_path / n) for n in ("a.dump", "ref." + fmt, "ours." + fmt, "r.dump", "o.dump"))
-            write_dump(a, dump)
-            subprocess.run([REF, "autosave", dump, ref_file], check=True)
-            image_io.convert_and_save_image(a, our_file)
-            subprocess.run([REF, "load", ref_file, d1], check=True)
-            subprocess.run([REF, "load", our_file, d2], check=True)
-            want, got = read_dump(d1), read_dump(d2)
-            assert got.dtype == want.dtype and got.shape == want.shape, (fmt, shape, src, got.dtype, want.dtype)
-            assert np.array_equal(got.view(np.uint8), want.view(np.uint8)), (fmt, shape, src)
+            our_file = str(tmp_path / ("img." + fmt))
+            image_io.convert_and_save_image(random_image(src, shape, 3), our_file)
+            assert file_sha(our_file) == reference()["autosave"][case_id(fmt, src, shape)], (fmt, shape, src)
 
 
-@have_ref
-def test_load_and_convert_of_the_reference_images(tmp_path):
-    """apps/images/gray_small.pgm and the camera_pipe colour matrices, loaded into every type the harnesses ask for."""
-    images = "/root/reference/apps/images"
-    if not os.path.isdir(images):
-        pytest.skip("reference images not present")
+def test_load_and_convert_of_the_reference_images():
+    """apps/images/gray_small.pgm (its first rows) and the camera_pipe colour matrices, loaded into every type the
+    harnesses ask for."""
     for name, types in (("gray_small.pgm", ("u8", "u16", "f32")), ("matrix_3200.mat", ("f32",)), ("matrix_7000.mat", ("f32", "f64"))):
         for t in types:
-            out = str(tmp_path / "x.dump")
-            subprocess.run([REF, "loadconv", os.path.join(images, name), t, out], check=True)
-            got = image_io.load_and_convert_image(os.path.join(images, name), NAMES[t])
-            want = read_dump(out)
-            assert got.dtype == want.dtype and np.array_equal(got, want), (name, t)
+            got = image_io.load_and_convert_image(os.path.join(IMAGES, name), NAMES[t])
+            want = reference()["load_and_convert"][f"{name}:{t}"]
+            assert TNAME[got.dtype] == want["dtype"] and list(got.shape) == want["shape"], (name, t)
+            assert sha(got) == want["sha256"], (name, t)
 
 
 def test_golden_files_decode_identically():
@@ -218,12 +187,11 @@ def test_png_codec_round_trip_and_cross_check(tmp_path):
 
 
 def test_reference_png_images_decode_the_same_both_ways():
-    """The reference's small sample images (apps/images/*_small*.png: 8-bit gray and RGB, 16-bit RGB, 16-bit Bayer raw)
-    through the pure-Python decoder and through OpenCV; gray_small.png must equal gray_small.pgm, which the reference's
-    own reader decodes (test_load_and_convert_of_the_reference_images)."""
-    images = "/root/reference/apps/images"
-    if not os.path.isdir(images):
-        pytest.skip("reference images not present")
+    """The reference's small sample images (apps/images/*_small*.png: 8-bit gray and RGB, 16-bit RGB, 16-bit Bayer raw;
+    their first rows, as filtered in the reference's files) through the pure-Python decoder and through OpenCV;
+    gray_small.png must equal gray_small.pgm, which the reference's own reader decodes
+    (test_load_and_convert_of_the_reference_images)."""
+    images = IMAGES
     try:
         import cv2  # noqa: F401
     except Exception:
@@ -240,18 +208,18 @@ def test_reference_png_images_decode_the_same_both_ways():
     assert np.array_equal(image_io.load(os.path.join(images, "gray_small.png")), image_io.load(os.path.join(images, "gray_small.pgm")))
 
 
-@have_ref
-@pytest.mark.parametrize("dtype,shape", [(np.uint8, (9, 14)), (np.uint16, (3, 9, 14)), (np.float32, (4, 5, 6)), (np.int32, (7,)),
-                                         (np.float64, (2, 3, 4, 5)), (np.uint8, (6, 3, 4)), (np.int16, (1, 2, 8, 9))])
+TIFF_CASES = [(np.uint8, (9, 14)), (np.uint16, (3, 9, 14)), (np.float32, (4, 5, 6)), (np.int32, (7,)), (np.float64, (2, 3, 4, 5)),
+              (np.uint8, (6, 3, 4)), (np.int16, (1, 2, 8, 9))]
+
+
+@pytest.mark.parametrize("dtype,shape", TIFF_CASES)
 def test_tiff_writer_is_byte_identical(dtype, shape, tmp_path):
     """The reference writes (uncompressed, planar) TIFF and cannot read it back; ours must produce the same bytes —
     including the rule that folds a third dimension below 5 into the channel count."""
     a = random_image(dtype, shape, 11)
-    dump, ref_file, our_file = (str(tmp_path / n) for n in ("a.dump", "ref.tiff", "ours.tiff"))
-    write_dump(a, dump)
-    subprocess.run([REF, "save", dump, ref_file], check=True)
+    our_file = str(tmp_path / "ours.tiff")
     image_io.save(a, our_file)
-    assert open(our_file, "rb").read() == open(ref_file, "rb").read()
+    assert file_sha(our_file) == reference()["tiff"][case_id("tiff", dtype, shape)]
     with pytest.raises(ValueError):
         image_io.load(our_file)
 
@@ -261,13 +229,7 @@ def test_natural_image_flow_like_process_cpp(tmp_path):
     filter (the CPU oracle stands in for it here — the GPU parity tests cover the filter itself), convert_and_save_image
     to a 16-bit PNG, reload: the file holds exactly the filter's output, and an 8-bit source enters as x * 257."""
     from oracle import pyoracle
-    images = "/root/reference/apps/images"
-    src = os.path.join(images, "rgb_small.png")
-    if not os.path.exists(src):
-        yy, xx = np.mgrid[0:48, 0:64]
-        rgb = np.stack([(np.sin(xx / 6.0) * 100 + 128), (np.cos(yy / 5.0) * 90 + 120), ((xx + yy) * 2 % 256)]).astype(np.uint8)
-        src = str(tmp_path / "synthetic.png")
-        image_io.save(rgb, src)
+    src = os.path.join(IMAGES, "rgb_small.png")
     native = image_io.load(src)
     assert native.dtype == np.uint8 and native.ndim == 3 and native.shape[0] == 3
     frame = image_io.load_and_convert_image(src, np.uint16)

@@ -1,5 +1,22 @@
-"""Shared helpers for the parity tests: seeded synthetic frames and C-ABI call wrappers."""
+"""Shared helpers for the parity tests: seeded synthetic frames, C-ABI call wrappers, and the digests of what the
+reference computed on the tests' inputs (tests/golden/reference_digests.json, tests/golden/make_reference_golden.py)."""
+import functools
+import hashlib
+import json
+import os
+
 import numpy as np
+
+
+@functools.lru_cache(maxsize=None)
+def reference():
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")) as f:
+        return json.load(f)
+
+
+def sha(data):
+    """SHA-256 of a byte string, or of an array's elements in C order."""
+    return hashlib.sha256(data if isinstance(data, bytes) else np.ascontiguousarray(data).tobytes()).hexdigest()
 
 
 def u16_frame(shape, seed, bits=16):
