@@ -167,6 +167,30 @@ int run_conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffe
         (r = hb::acquire_input(bias, kBias, &db)) || (r = hb::acquire_output(relu, kOut, &dout)))
         return r;
     cudaStream_t s = hb::stream();
+    // Both contractions move every operand and the output in float4s.  A caller's device buffer that is not 16-byte
+    // aligned (a wrapped tensor view at an odd element offset) is staged through pooled scratch, which is.
+    hb::Scratch staging;
+    float *user_out = nullptr;
+    const size_t out_bytes = (size_t)N * H * W * CO * sizeof(float);
+    {
+        const size_t bytes[3] = {(size_t)N * (H + 2) * (W + 2) * CI * sizeof(float), (size_t)CO * 9 * CI * sizeof(float),
+                                 (size_t)CO * sizeof(float)};
+        void **ptrs[3] = {&din, &df, &db};
+        for (int i = 0; i < 3; i++) {
+            if (((uintptr_t)*ptrs[i] & 15) == 0) continue;
+            void *a = staging.get<uint8_t>(bytes[i]);
+            if (!a) return hb::fail(halide_error_code_device_malloc_failed, "conv_layer: staging allocation failed");
+            if ((r = hb::check_cuda(cudaMemcpyAsync(a, *ptrs[i], bytes[i], cudaMemcpyDeviceToDevice, s), "conv_layer staging copy",
+                                    halide_error_code_device_run_failed)))
+                return r;
+            *ptrs[i] = a;
+        }
+        if ((uintptr_t)dout & 15) {
+            user_out = (float *)dout;
+            if (!(dout = staging.get<uint8_t>(out_bytes)))
+                return hb::fail(halide_error_code_device_malloc_failed, "conv_layer: staging allocation failed");
+        }
+    }
     {
         hb::CallTimer timer(s);
         if (g_use_tc) {
@@ -177,6 +201,9 @@ int run_conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffe
                       (float *)dout);
         }
     }
+    if (user_out && (r = hb::check_cuda(cudaMemcpyAsync(user_out, dout, out_bytes, cudaMemcpyDeviceToDevice, s), "conv_layer staging copy",
+                                        halide_error_code_device_run_failed)))
+        return r;
     if ((r = hb::check_cuda(cudaGetLastError(), "conv_layer launch", halide_error_code_device_run_failed))) return r;
     hb::mark_output_written(relu);
     return 0;

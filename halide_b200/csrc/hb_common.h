@@ -52,6 +52,8 @@ struct PerDeviceOnce {
 // ---- device scratch (callee-owned intermediates; pooled, src/runtime/cuda.cpp:760-870 analogue) ---
 void *scratch_alloc(size_t bytes);  // returns nullptr on failure (caller maps to -16)
 void scratch_free(void *p);         // stream-ordered: safe to call right after the last launch
+// Under halide_b200_debug_fill_allocations, memset a fresh device block to the fill byte on `s` (no-op when off).
+void *debug_fill(void *p, size_t bytes, cudaStream_t s);
 
 struct Scratch {  // frees everything it handed out when the filter call returns
     static constexpr int kMax = 48;

@@ -23,6 +23,7 @@ namespace {
 
 std::atomic<halide_error_handler_t> g_handler{nullptr};
 std::atomic<uint64_t> g_launches{0};
+std::atomic<int> g_fill_byte{-1};  // halide_b200_debug_fill_allocations: -1 = off
 thread_local cudaStream_t t_stream = nullptr;
 
 // ---- device allocation pool ------------------------------------------------------------------
@@ -49,7 +50,7 @@ struct Pool {
                 free_blocks.erase(it);
                 cached_bytes -= bytes;
                 live[p] = bytes;
-                return p;
+                return hb::debug_fill(p, bytes, t_stream);
             }
         }
         void *p = nullptr;
@@ -62,9 +63,11 @@ struct Pool {
                 return nullptr;
             }
         }
-        std::lock_guard<std::mutex> lock(mu);
-        live[p] = bytes;
-        return p;
+        {
+            std::lock_guard<std::mutex> lock(mu);
+            live[p] = bytes;
+        }
+        return hb::debug_fill(p, bytes, t_stream);
     }
     void free(void *p) {
         if (!p) return;
@@ -516,6 +519,11 @@ void *scratch_alloc(size_t bytes) {
 void scratch_free(void *p) {
     pool().free(p);
 }
+void *debug_fill(void *p, size_t bytes, cudaStream_t s) {
+    const int b = g_fill_byte.load(std::memory_order_relaxed);
+    if (p && b >= 0) cudaMemsetAsync(p, b, bytes, s);
+    return p;
+}
 
 static const char *kind(const ArgSpec &s) {
     return s.is_output ? "Output" : "Input";
@@ -781,6 +789,10 @@ uint64_t halide_b200_kernel_launch_count(void) {
 }
 const char *halide_b200_target(void) {
     return "x86-64-linux-cuda-cuda_capability_100-b200_native";
+}
+
+void halide_b200_debug_fill_allocations(int byte) {
+    g_fill_byte.store(byte >= 0 && byte <= 255 ? byte : -1);
 }
 
 void halide_b200_set_timing(int enable) {

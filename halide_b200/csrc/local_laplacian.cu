@@ -162,6 +162,7 @@ int get_lut(Plan &p, cudaStream_t s) {
         cudaGetLastError();
         return hb::fail(halide_error_code_device_malloc_failed, "local_laplacian: remap table allocation failed");
     }
+    hb::debug_fill(lut, ((size_t)n + 3) / 4 * 16, s);
     HB_LAUNCH("ll_lut", ll_lut_kernel, (n + 255) / 256, 256, 0, s, lut, p.f.lut_half, p.alpha);
     if (cudaStreamSynchronize(s) != cudaSuccess) {
         cudaGetLastError();

@@ -307,6 +307,11 @@ void halide_b200_nl_means_variant(int variant);
 void halide_b200_stencil_chain_variant(int variant);
 /* conv_layer: 1 = tcgen05/TMEM/TMA implicit GEMM (3xTF32 split), 0 = FP32 SIMT kernel (also HALIDE_B200_CONV=tc|simt). */
 void halide_b200_conv_use_tensor_cores(int enable);
+/* Test hook: byte in 0..255 makes every device block the library hands out (buffer device_malloc, filter scratch,
+ * the local_laplacian remap table) start filled with that byte, memset on the calling thread's stream before the
+ * block is returned, so an unwritten output element or unwritten scratch shows up as a wrong value instead of
+ * whatever the recycled block last held; -1 (the default) turns it off. */
+void halide_b200_debug_fill_allocations(int byte);
 /* Device self-test of the fast kernels' arithmetic shortcuts; returns mismatches vs div.rn / cvt, or -1. */
 long long halide_b200_selftest_arith(unsigned long long n, unsigned long long seed);
 
