@@ -49,3 +49,15 @@ def camera_pipe(input, matrix_3200, matrix_7000, color_temp, gamma, contrast, sh
 def conv_layer(input, filter, bias, relu):
     """apps/conv_layer/conv_layer_generator.cpp: 3x3 conv + bias + relu, fixed shapes (N5 CI128 CO128 100x80), f32."""
     return check(lib.conv_layer(input.ptr, filter.ptr, bias.ptr, relu.ptr))
+
+
+def harris(input, output):
+    """apps/harris/harris_generator.cpp: Harris corner response, float32 (x, y, c) -> (x, y).  No boundary condition:
+    the input must cover the output box grown by 2 in x and y, and channels 0..2."""
+    return check(lib.harris(input.ptr, output.ptr))
+
+
+def unsharp(input, output):
+    """apps/unsharp/unsharp_generator.cpp (sigma 1.5): unsharp mask, float32 (x, y, c) -> (x, y, c).  The input is
+    edge-clamped for the luma blur and must cover the output's (x, y, c) box."""
+    return check(lib.unsharp(input.ptr, output.ptr))

@@ -28,6 +28,21 @@ def u16(shape, dev, g):
     return torch.randint(-32768, 32768, shape, dtype=torch.int16, device=dev, generator=g).view(torch.uint16)
 
 
+def gpu_info():
+    """Card name, power limit and max SM clock (nvidia-smi query, read-only) and the SM count of cuda:0."""
+    import subprocess
+    name, power, mhz = "unknown", "unknown", 0
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader,nounits"],
+                           capture_output=True, text=True, timeout=30).stdout.splitlines()[0]
+        name, power, mhz = (v.strip() for v in q.split(","))
+        power, mhz = f"{float(power):.0f} W", int(float(mhz))
+    except Exception:
+        pass
+    return {"name": name, "power_limit": power, "max_sm_mhz": mhz or 1965,
+            "sms": torch.cuda.get_device_properties(0).multi_processor_count}
+
+
 LAST_KERNELS = {}
 
 
@@ -163,6 +178,43 @@ def main():
             a = np.random.default_rng(0).integers(0, 65536, (3, 1080, 3840), dtype=np.uint16)
             report("local_laplacian", f"{W}x{H}x3 u16 levels 8", W * H, 12 * W * H, t, cpu_time(lambda: pyoracle.local_laplacian(a, 8, 1 / 7, 1.0)) * (W * H / (3840 * 1080)),
                    "3840x1080 band scaled by area")
+    if want("harris") or want("unsharp"):  # ---- harris / unsharp: the generators' estimate frame and 8K, f32
+        from oracle import pyoracle_apps
+        gpu = gpu_info()
+        # f32 flops per output pixel from the generators' expressions (apron recomputation not counted)
+        fl_gray = 3 + 2                                      # 3 mul, 2 add
+        fl_harris = (fl_gray + 2 * 11 + 3                    # gray; Ix, Iy: 6 mul + 5 add each; Ixx, Iyy, Ixy
+                     + 3 * 8 + 3 + 1 + 3)                    # three 9-term sums; det; trace; det - 0.04 trace^2
+        fl_unsharp = (fl_gray + 2 * 10                       # gray; blur_y, blur_x: 4 mul + 6 add each
+                      + 2 + 1 + 3)                           # sharpen; ratio (one divide); ratio * input for 3 channels
+        fp32_peak = gpu["sms"] * 128 * 2 * gpu["max_sm_mhz"] * 1e6
+        for name, bpp, fpp in (("harris", 16, fl_harris), ("unsharp", 24, fl_unsharp)):
+            if not want(name):
+                continue
+            for (W, H) in [(1536, 2560), (7680, 4320)]:
+                fn = getattr(filters, name)
+                # enough buffer sets that one rotation exceeds the 126 MB L2
+                sets = max(2, int(np.ceil(4 * 126e6 / (bpp * W * H))))
+                def mk():
+                    out_shape = (H, W) if name == "harris" else (3, H, W)
+                    ins = (3, H + 6, W + 6) if name == "harris" else (3, H, W)
+                    res = []
+                    for _ in range(sets):
+                        bo = HalideBuffer.from_torch(torch.zeros(out_shape, dtype=torch.float32, device=dev),
+                                                     mins=(3, 3) if name == "harris" else None)
+                        res.append((HalideBuffer.from_torch(torch.rand(ins, dtype=torch.float32, device=dev, generator=g)), bo))
+                    return res
+                t = time_gpu(mk, fn, 200 if W < 4000 else 50)
+                frac = 1 if W < 4000 else 4
+                pad = 6 if name == "harris" else 0
+                a = np.random.default_rng(0).random((3, H // frac + pad, W + pad), dtype=np.float32)
+                t_cpu = cpu_time(lambda: getattr(pyoracle_apps, name)(a)) * frac
+                bound = "hbm" if bpp / (pk * 1e9) >= fpp / fp32_peak else "fp32"
+                report(name, f"{W + 6}x{H + 6}x3 f32 -> {W}x{H} at (3,3)" if name == "harris" else f"{W}x{H}x3 f32", W * H, bpp * W * H, t,
+                       t_cpu, "full frame" if frac == 1 else "1/4 of the frame x4", bound=bound, flops=fpp * W * H,
+                       note=f"{fpp} flop/px, {bpp} B/px; {sets} buffer sets; fp32 peak {fp32_peak / 1e12:.1f} TFLOP/s from "
+                            f"{gpu['sms']} SMs at {gpu['max_sm_mhz']} MHz; {gpu['name']}, power limit {gpu['power_limit']}")
+                rows[-1]["fp32_frac"] = fpp * W * H / t / fp32_peak
     json.dump(rows, open(os.path.join(ROOT, "gpurun_out", "bench_all.json"), "w"), indent=1)
 
 

@@ -19,6 +19,10 @@ FILTERS = {
                    "struct halide_buffer_t *input, struct halide_buffer_t *filter, struct halide_buffer_t *bias, struct halide_buffer_t *relu", True),
     "camera_pipe": ("apps/camera_pipe/camera_pipe_generator.cpp:218-238,622",
                     "struct halide_buffer_t *input, struct halide_buffer_t *matrix_3200, struct halide_buffer_t *matrix_7000, float color_temp, float gamma, float contrast, float sharpen_strength, int32_t blackLevel, int32_t whiteLevel, struct halide_buffer_t *processed", True),
+    "harris": ("apps/harris/harris_generator.cpp:15-16,131",
+               "struct halide_buffer_t *input, struct halide_buffer_t *output", True),
+    "unsharp": ("apps/unsharp/unsharp_generator.cpp:7-10,114",
+                "struct halide_buffer_t *input, struct halide_buffer_t *output", True),
 }
 
 
