@@ -18,6 +18,8 @@
 //                   4 pixels per thread (float4 in / float4 out), 8 shared 8-byte corner loads per pixel.
 // Grid layout in HBM: [cell_y][cell_x][z][2] f32 — the (z, z+1) x (value, weight) quad a pixel
 // needs at one corner is 16 contiguous bytes.
+#include "../../include/bilateral_grid.h"
+#include "../../include/bilateral_grid_auto_schedule.h"
 #include "hb_common.h"
 #include "hl_math.cuh"
 
@@ -210,29 +212,23 @@ __global__ void __launch_bounds__(256) bg_slice_kernel(BGParams p) {
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_float, 32, 2, false};
-const hb::ArgSpec kOut = {"bilateral_grid", halide_type_float, 32, 2, true};
-int64_t est_i[2][2] = {{0, 1536}, {0, 2560}};
-const int64_t *const est_ptrs[4] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1]};
-halide_scalar_value_t sv_rsigma;
-struct InitScalars {
-    InitScalars() { sv_rsigma.u.i64 = 0; sv_rsigma.u.f32 = 0.1f; }
-} init_scalars;
+const hb::BufferEstimates est({0, 1536, 0, 2560});
+const halide_scalar_value_t sv_rsigma = hb::scalar(0.1f);
 const halide_filter_argument_t kArgs[3] = {
-    {"input", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"input", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
     {"r_sigma", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv_rsigma, nullptr},
-    {"bilateral_grid", halide_argument_kind_output_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"bilateral_grid", halide_argument_kind_output_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
 };
-const halide_filter_metadata_t kMeta = {1, 3, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "bilateral_grid"};
-const halide_filter_metadata_t kMetaAuto = {1, 3, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "bilateral_grid_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[2];
 
 inline int fdiv(int a, int b) {  // floor division, b > 0
     int q = a / b;
     return (a % b != 0 && a < 0) ? q - 1 : q;
 }
 
-int run_bilateral_grid(halide_buffer_t *input, float r_sigma, halide_buffer_t *output) {
+}  // namespace
+
+extern "C" int bilateral_grid(halide_buffer_t *input, float r_sigma, halide_buffer_t *output) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(output, kOut))) return r;
@@ -314,23 +310,5 @@ int run_bilateral_grid(halide_buffer_t *input, float r_sigma, halide_buffer_t *o
     return 0;
 }
 
-}  // namespace
-
-extern "C" int bilateral_grid(halide_buffer_t *input, float r_sigma, halide_buffer_t *output) {
-    return run_bilateral_grid(input, r_sigma, output);
-}
-extern "C" int bilateral_grid_argv(void **args) {
-    return run_bilateral_grid((halide_buffer_t *)args[0], *(float *)args[1], (halide_buffer_t *)args[2]);
-}
-extern "C" const halide_filter_metadata_t *bilateral_grid_metadata(void) {
-    return &kMeta;
-}
-extern "C" int bilateral_grid_auto_schedule(halide_buffer_t *input, float r_sigma, halide_buffer_t *output) {
-    return run_bilateral_grid(input, r_sigma, output);
-}
-extern "C" int bilateral_grid_auto_schedule_argv(void **args) {
-    return bilateral_grid_argv(args);
-}
-extern "C" const halide_filter_metadata_t *bilateral_grid_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(bilateral_grid, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(bilateral_grid, kArgs)

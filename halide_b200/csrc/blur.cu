@@ -15,6 +15,7 @@
 //     strips sized to fill the resident warps a whole number of times.  29.8 us at 8K (68 % of the measured HBM peak).
 //   * blur3x3_u16_kernel — any alignment: a lane owns 8 pixels, aligned 16-byte loads realigned by funnel shifts, the
 //     2-pixel horizontal apron from the neighbouring lane by shuffle.  Bound by the integer pipe (49 us at 8K).
+#include "../../include/halide_blur.h"
 #include "hb_common.h"
 
 namespace {
@@ -291,14 +292,11 @@ __global__ void __launch_bounds__(32 * kQuadWarps) blur3x3_u16_quad_kernel(BlurA
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_uint, 16, 2, false};
-const hb::ArgSpec kOut = {"blur_y", halide_type_uint, 16, 2, true};
-
 const halide_filter_argument_t kArgs[2] = {
     {"input", halide_argument_kind_input_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, nullptr},
     {"blur_y", halide_argument_kind_output_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, nullptr},
 };
-const halide_filter_metadata_t kMeta = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "halide_blur"};
+const auto &kIn = kArgs[0], &kOut = kArgs[1];
 
 }  // namespace
 
@@ -407,10 +405,4 @@ extern "C" void halide_b200_blur_force_general(int enable) {
     g_force_general = enable;
 }
 
-extern "C" int halide_blur_argv(void **args) {
-    return halide_blur((halide_buffer_t *)args[0], (halide_buffer_t *)args[1]);
-}
-
-extern "C" const halide_filter_metadata_t *halide_blur_metadata(void) {
-    return &kMeta;
-}
+HB_EXPORT_FILTER(halide_blur, kArgs)

@@ -13,6 +13,8 @@
 //   camera_pipe_kernel one 64x32 output tile per block:
 //        raw (+apron) -> smem -> denoised -> g_r/g_b at half resolution -> demosaic + matrix + curve (u8, tile+1)
 //        -> unsharp mask -> 4 pixels per thread stored as one 32-bit word per channel
+#include "../../include/camera_pipe.h"
+#include "../../include/camera_pipe_auto_schedule.h"
 #include "hb_common.h"
 #include "hl_math.cuh"
 
@@ -227,45 +229,33 @@ __global__ void __launch_bounds__(256) camera_pipe_kernel(CPParams p) {
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_uint, 16, 2, false};
-const hb::ArgSpec kM32 = {"matrix_3200", halide_type_float, 32, 2, false};
-const hb::ArgSpec kM70 = {"matrix_7000", halide_type_float, 32, 2, false};
-const hb::ArgSpec kOut = {"processed", halide_type_uint, 8, 3, true};
-
-int64_t est_in[2][2] = {{0, 2592}, {0, 1968}}, est_m[2][2] = {{0, 4}, {0, 3}}, est_out[3][2] = {{0, 2592}, {0, 1968}, {0, 3}};
-const int64_t *const est_in_p[4] = {&est_in[0][0], &est_in[0][1], &est_in[1][0], &est_in[1][1]};
-const int64_t *const est_m_p[4] = {&est_m[0][0], &est_m[0][1], &est_m[1][0], &est_m[1][1]};
-const int64_t *const est_out_p[6] = {&est_out[0][0], &est_out[0][1], &est_out[1][0], &est_out[1][1], &est_out[2][0], &est_out[2][1]};
-halide_scalar_value_t sv[6];
-struct InitScalars {
-    InitScalars() {
-        for (auto &v : sv) v.u.i64 = 0;
-        sv[0].u.f32 = 3700; sv[1].u.f32 = 2.0f; sv[2].u.f32 = 50; sv[3].u.f32 = 1.0f; sv[4].u.i32 = 25; sv[5].u.i32 = 1023;
-    }
-} init_scalars;
+const hb::BufferEstimates est_in({0, 2592, 0, 1968}), est_m({0, 4, 0, 3});
+const hb::BufferEstimates est_out({0, 2592, 0, 1968, 0, 3});
+const halide_scalar_value_t sv[6] = {hb::scalar(3700.0f), hb::scalar(2.0f), hb::scalar(50.0f), hb::scalar(1.0f), hb::scalar(25),
+                                     hb::scalar(1023)};
 const halide_filter_argument_t kArgs[10] = {
-    {"input", halide_argument_kind_input_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_in_p},
-    {"matrix_3200", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_m_p},
-    {"matrix_7000", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_m_p},
+    {"input", halide_argument_kind_input_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_in.p},
+    {"matrix_3200", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_m.p},
+    {"matrix_7000", halide_argument_kind_input_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_m.p},
     {"color_temp", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv[0], nullptr},
     {"gamma", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv[1], nullptr},
     {"contrast", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv[2], nullptr},
     {"sharpen_strength", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv[3], nullptr},
     {"blackLevel", halide_argument_kind_input_scalar, 0, {halide_type_int, 32, 0}, nullptr, nullptr, nullptr, &sv[4], nullptr},
     {"whiteLevel", halide_argument_kind_input_scalar, 0, {halide_type_int, 32, 0}, nullptr, nullptr, nullptr, &sv[5], nullptr},
-    {"processed", halide_argument_kind_output_buffer, 3, {halide_type_uint, 8, 0}, nullptr, nullptr, nullptr, nullptr, est_out_p},
+    {"processed", halide_argument_kind_output_buffer, 3, {halide_type_uint, 8, 0}, nullptr, nullptr, nullptr, nullptr, est_out.p},
 };
-const halide_filter_metadata_t kMeta = {1, 10, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "camera_pipe"};
-const halide_filter_metadata_t kMetaAuto = {1, 10, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "camera_pipe_auto_schedule"};
+const auto &kIn = kArgs[0], &kM32 = kArgs[1], &kM70 = kArgs[2], &kOut = kArgs[9];
 
 inline int fdiv(int a, int b) {
     int q = a / b;
     return (a % b != 0 && ((a < 0) != (b < 0))) ? q - 1 : q;
 }
 
-int run_camera_pipe(halide_buffer_t *input, halide_buffer_t *m3200, halide_buffer_t *m7000, float color_temp, float gamma,
-                    float contrast, float sharpen_strength, int blackLevel, int whiteLevel, halide_buffer_t *out) {
+}  // namespace
+
+extern "C" int camera_pipe(halide_buffer_t *input, halide_buffer_t *m3200, halide_buffer_t *m7000, float color_temp, float gamma,
+                           float contrast, float sharpen_strength, int32_t blackLevel, int32_t whiteLevel, halide_buffer_t *out) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(m3200, kM32))) return r;
@@ -303,7 +293,7 @@ int run_camera_pipe(halide_buffer_t *input, halide_buffer_t *m3200, halide_buffe
     if ((r = hb::check_covers(input, kIn, 0, need_x0, need_x1 - need_x0 + 1))) return r;
     if ((r = hb::check_covers(input, kIn, 1, need_y0, need_y1 - need_y0 + 1))) return r;
     for (halide_buffer_t *m : {m3200, m7000}) {
-        const hb::ArgSpec &sp = m == m3200 ? kM32 : kM70;
+        const halide_filter_argument_t &sp = m == m3200 ? kM32 : kM70;
         if ((r = hb::check_covers(m, sp, 0, 0, 4)) || (r = hb::check_covers(m, sp, 1, 0, 3))) return r;
     }
     if ((r = hb::check_covers(out, kOut, 2, out->dim[2].min, out->dim[2].extent))) return r;
@@ -348,30 +338,5 @@ int run_camera_pipe(halide_buffer_t *input, halide_buffer_t *m3200, halide_buffe
     return 0;
 }
 
-}  // namespace
-
-extern "C" int camera_pipe(halide_buffer_t *input, halide_buffer_t *matrix_3200, halide_buffer_t *matrix_7000, float color_temp,
-                           float gamma, float contrast, float sharpen_strength, int32_t blackLevel, int32_t whiteLevel,
-                           halide_buffer_t *processed) {
-    return run_camera_pipe(input, matrix_3200, matrix_7000, color_temp, gamma, contrast, sharpen_strength, blackLevel, whiteLevel,
-                           processed);
-}
-extern "C" int camera_pipe_argv(void **a) {
-    return run_camera_pipe((halide_buffer_t *)a[0], (halide_buffer_t *)a[1], (halide_buffer_t *)a[2], *(float *)a[3], *(float *)a[4],
-                           *(float *)a[5], *(float *)a[6], *(int32_t *)a[7], *(int32_t *)a[8], (halide_buffer_t *)a[9]);
-}
-extern "C" const halide_filter_metadata_t *camera_pipe_metadata(void) {
-    return &kMeta;
-}
-extern "C" int camera_pipe_auto_schedule(halide_buffer_t *input, halide_buffer_t *matrix_3200, halide_buffer_t *matrix_7000,
-                                         float color_temp, float gamma, float contrast, float sharpen_strength, int32_t blackLevel,
-                                         int32_t whiteLevel, halide_buffer_t *processed) {
-    return run_camera_pipe(input, matrix_3200, matrix_7000, color_temp, gamma, contrast, sharpen_strength, blackLevel, whiteLevel,
-                           processed);
-}
-extern "C" int camera_pipe_auto_schedule_argv(void **a) {
-    return camera_pipe_argv(a);
-}
-extern "C" const halide_filter_metadata_t *camera_pipe_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(camera_pipe, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(camera_pipe, kArgs)

@@ -16,6 +16,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "../../include/conv_layer.h"
+#include "../../include/conv_layer_auto_schedule.h"
 #include "hb_common.h"
 
 // tcgen05 / TMEM / TMA implementation (conv_layer_tc.cu)
@@ -103,26 +105,18 @@ __global__ void __launch_bounds__(256) conv_layer_kernel(const float *__restrict
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_float, 32, 4, false};
-const hb::ArgSpec kFilt = {"filter", halide_type_float, 32, 4, false};
-const hb::ArgSpec kBias = {"bias", halide_type_float, 32, 1, false};
-const hb::ArgSpec kOut = {"relu", halide_type_float, 32, 4, true};
-
 // estimates = the fixed shapes (generator :52-68)
-int64_t e_zero = 0, e_ci = CI, e_co = CO, e_wp = W + 2, e_hp = H + 2, e_w = W, e_h = H, e_n = N, e_3 = 3;
-const int64_t *const est_in[8] = {&e_zero, &e_ci, &e_zero, &e_wp, &e_zero, &e_hp, &e_zero, &e_n};
-const int64_t *const est_f[8] = {&e_zero, &e_co, &e_zero, &e_3, &e_zero, &e_3, &e_zero, &e_ci};
-const int64_t *const est_b[2] = {&e_zero, &e_co};
-const int64_t *const est_out[8] = {&e_zero, &e_co, &e_zero, &e_w, &e_zero, &e_h, &e_zero, &e_n};
+const hb::BufferEstimates est_in({0, CI, 0, W + 2, 0, H + 2, 0, N});
+const hb::BufferEstimates est_f({0, CO, 0, 3, 0, 3, 0, CI});
+const hb::BufferEstimates est_b({0, CO});
+const hb::BufferEstimates est_out({0, CO, 0, W, 0, H, 0, N});
 const halide_filter_argument_t kArgs[4] = {
-    {"input", halide_argument_kind_input_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_in},
-    {"filter", halide_argument_kind_input_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_f},
-    {"bias", halide_argument_kind_input_buffer, 1, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_b},
-    {"relu", halide_argument_kind_output_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_out},
+    {"input", halide_argument_kind_input_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_in.p},
+    {"filter", halide_argument_kind_input_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_f.p},
+    {"bias", halide_argument_kind_input_buffer, 1, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_b.p},
+    {"relu", halide_argument_kind_output_buffer, 4, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_out.p},
 };
-const halide_filter_metadata_t kMeta = {1, 4, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "conv_layer"};
-const halide_filter_metadata_t kMetaAuto = {1, 4, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "conv_layer_auto_schedule"};
+const auto &kIn = kArgs[0], &kFilt = kArgs[1], &kBias = kArgs[2], &kOut = kArgs[3];
 
 struct Shape {
     int ext[4];
@@ -130,7 +124,7 @@ struct Shape {
 // the generator's set_bounds / set_stride constraints (:35-50)
 const Shape kInShape = {{CI, W + 2, H + 2, N}}, kFiltShape = {{CO, 3, 3, CI}}, kOutShape = {{CO, W, H, N}};
 
-int check_fixed(const halide_buffer_t *b, const hb::ArgSpec &spec, const int *ext, int nd) {
+int check_fixed(const halide_buffer_t *b, const halide_filter_argument_t &spec, const int *ext, int nd) {
     int64_t stride = 1;
     for (int d = 0; d < nd; d++) {
         if (b->dim[d].min != 0 || b->dim[d].extent != ext[d] || b->dim[d].stride != stride) {
@@ -143,7 +137,9 @@ int check_fixed(const halide_buffer_t *b, const hb::ArgSpec &spec, const int *ex
     return 0;
 }
 
-int run_conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffer_t *bias, halide_buffer_t *relu) {
+}  // namespace
+
+extern "C" int conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffer_t *bias, halide_buffer_t *relu) {
     int r;
     if ((r = hb::check_arg(input, kIn)) || (r = hb::check_arg(filter, kFilt)) || (r = hb::check_arg(bias, kBias)) ||
         (r = hb::check_arg(relu, kOut)))
@@ -209,26 +205,8 @@ int run_conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffe
     return 0;
 }
 
-}  // namespace
-
-extern "C" int conv_layer(halide_buffer_t *input, halide_buffer_t *filter, halide_buffer_t *bias, halide_buffer_t *relu) {
-    return run_conv_layer(input, filter, bias, relu);
-}
-extern "C" int conv_layer_argv(void **a) {
-    return run_conv_layer((halide_buffer_t *)a[0], (halide_buffer_t *)a[1], (halide_buffer_t *)a[2], (halide_buffer_t *)a[3]);
-}
-extern "C" const halide_filter_metadata_t *conv_layer_metadata(void) {
-    return &kMeta;
-}
-extern "C" int conv_layer_auto_schedule(halide_buffer_t *input, halide_buffer_t *filter, halide_buffer_t *bias, halide_buffer_t *relu) {
-    return run_conv_layer(input, filter, bias, relu);
-}
-extern "C" int conv_layer_auto_schedule_argv(void **a) {
-    return conv_layer_argv(a);
-}
-extern "C" const halide_filter_metadata_t *conv_layer_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(conv_layer, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(conv_layer, kArgs)
 
 extern "C" void halide_b200_conv_use_tensor_cores(int enable) {
     g_use_tc = enable != 0;

@@ -12,6 +12,8 @@
 // One fused kernel, like the reference's GPU schedule: a block stages its 32x32 tile plus a 2-pixel apron once
 // (hb_tile.cuh), then gray, the gradient products and the 3x3 sums live in shared memory and registers only.
 // Algorithmic traffic is 16 B/px (12 in, 4 out) against ~70 flops/px.
+#include "../../include/harris.h"
+#include "../../include/harris_auto_schedule.h"
 #include "hb_common.h"
 #include "hb_tile.cuh"
 
@@ -87,21 +89,17 @@ __global__ void __launch_bounds__(NT) harris_kernel(HarrisParams q) {
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_float, 32, 3, false};
-const hb::ArgSpec kOut = {"output", halide_type_float, 32, 2, true};
-int64_t est_i[3][2] = {{0, 1536}, {0, 2560}, {0, 3}};
-int64_t est_o[2][2] = {{3, 1530}, {3, 2554}};  // output.dim(d).set_estimate(3, k - 6) (generator :70-71)
-const int64_t *const est_in[6] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1], &est_i[2][0], &est_i[2][1]};
-const int64_t *const est_out[4] = {&est_o[0][0], &est_o[0][1], &est_o[1][0], &est_o[1][1]};
+const hb::BufferEstimates est_in({0, 1536, 0, 2560, 0, 3});
+const hb::BufferEstimates est_out({3, 1530, 3, 2554});  // output.dim(d).set_estimate(3, k - 6) (generator :70-71)
 const halide_filter_argument_t kArgs[2] = {
-    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_in},
-    {"output", halide_argument_kind_output_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_out},
+    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_in.p},
+    {"output", halide_argument_kind_output_buffer, 2, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_out.p},
 };
-const halide_filter_metadata_t kMeta = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "harris"};
-const halide_filter_metadata_t kMetaAuto = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "harris_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[1];
 
-int run_harris(halide_buffer_t *input, halide_buffer_t *output) {
+}  // namespace
+
+extern "C" int harris(halide_buffer_t *input, halide_buffer_t *output) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(output, kOut))) return r;
@@ -143,23 +141,5 @@ int run_harris(halide_buffer_t *input, halide_buffer_t *output) {
     return 0;
 }
 
-}  // namespace
-
-extern "C" int harris(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_harris(input, output);
-}
-extern "C" int harris_argv(void **args) {
-    return run_harris((halide_buffer_t *)args[0], (halide_buffer_t *)args[1]);
-}
-extern "C" const halide_filter_metadata_t *harris_metadata(void) {
-    return &kMeta;
-}
-extern "C" int harris_auto_schedule(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_harris(input, output);
-}
-extern "C" int harris_auto_schedule_argv(void **args) {
-    return harris_argv(args);
-}
-extern "C" const halide_filter_metadata_t *harris_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(harris, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(harris, kArgs)

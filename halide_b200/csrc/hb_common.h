@@ -11,6 +11,9 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <type_traits>
+#include <utility>
+
 #include "../../include/halide_b200_runtime.h"
 
 namespace hb {
@@ -72,27 +75,21 @@ struct Scratch {  // frees everything it handed out when the filter call returns
 };
 
 // ---- buffer validation -----------------------------------------------------------------------
-struct ArgSpec {
-    const char *name;  // "Input buffer input", "Output buffer output" style prefix is added by fail()
-    uint8_t code;      // halide_type_uint / halide_type_float ...
-    uint8_t bits;
-    int dimensions;
-    bool is_output;
-};
-
+// A buffer is checked against its argument's metadata record: name, type code/bits, dimensions, and input vs
+// output from the kind.  So F enforces what F_metadata() reports.
 inline bool is_bounds_query(const halide_buffer_t *b) {
     return b->host == nullptr && b->device == 0;  // HalideRuntime.h:1851-1853
 }
 
 // null → -12, type → -3, dimensions → -43.  (Extent/stride checks need the required region and
 // are done by check_shape after the bounds-query early-out, as in the generated prologue.)
-int check_arg(const halide_buffer_t *b, const ArgSpec &spec);
+int check_arg(const halide_buffer_t *b, const halide_filter_argument_t &spec);
 
 // negative extent → -28, |extent*stride| and allocation size limits → -5/-6, stride[0] != 1 → -8.
-int check_shape(const halide_buffer_t *b, const ArgSpec &spec);
+int check_shape(const halide_buffer_t *b, const halide_filter_argument_t &spec);
 
 // required [min, min+extent) per dimension must lie inside the buffer → else -4.
-int check_covers(const halide_buffer_t *b, const ArgSpec &spec, int dim, int req_min, int req_extent);
+int check_covers(const halide_buffer_t *b, const halide_filter_argument_t &spec, int dim, int req_min, int req_extent);
 
 // Bounds-query answer: write min/extent and dense strides (src/AddImageChecks.cpp:386-436).
 void propose_shape(halide_buffer_t *b, const int *mins, const int *extents);
@@ -101,15 +98,77 @@ void propose_shape(halide_buffer_t *b, const int *mins, const int *extents);
 // Make the buffer's contents available on the device and return the device address of the
 // element at the mins.  Inputs: allocate + H2D when host_dirty or no device allocation yet.
 // Outputs: allocate only.  Returns 0 or a negative halide_error_code_t.
-int acquire_input(halide_buffer_t *b, const ArgSpec &spec, void **dev_ptr);
-int acquire_output(halide_buffer_t *b, const ArgSpec &spec, void **dev_ptr);
+int acquire_input(halide_buffer_t *b, const halide_filter_argument_t &spec, void **dev_ptr);
+int acquire_output(halide_buffer_t *b, const halide_filter_argument_t &spec, void **dev_ptr);
 void mark_output_written(halide_buffer_t *b);
 
 inline size_t elem_bytes(const halide_buffer_t *b) {
     return (b->type.bits + 7) / 8;
 }
 
+// ---- exported surface: Halide's F_argv / F_metadata convention (src/CodeGen_C.cpp:675-721) ---------------------
+constexpr const char *kTarget = "x86-64-linux-cuda-cuda_capability_100-b200_native";
+
+// F_argv(args): args[i] points at argument i; a buffer argument is passed as the pointer itself.
+template<typename T>
+T argv_arg(void *a) {
+    if constexpr (std::is_pointer_v<T>) return (T)a;
+    else return *(T *)a;
+}
+template<typename... A, size_t... I>
+int call_argv(int (*f)(A...), void **args, std::index_sequence<I...>) {
+    return f(argv_arg<A>(args[I])...);
+}
+template<typename... A>
+int call_argv(int (*f)(A...), void **args) {
+    return call_argv(f, args, std::index_sequence_for<A...>{});
+}
+
+// A buffer argument's estimates in the metadata's layout: one pointer per value, {min, extent} per dimension.
+template<size_t N>
+struct BufferEstimates {
+    int64_t v[N] = {};
+    const int64_t *p[N] = {};
+    constexpr BufferEstimates(const int64_t (&mins_extents)[N]) {
+        for (size_t i = 0; i < N; i++) {
+            v[i] = mins_extents[i];
+            p[i] = &v[i];
+        }
+    }
+    BufferEstimates(const BufferEstimates &) = delete;
+};
+
+// Scalar metadata cells (the unused upper bytes are zero).
+inline halide_scalar_value_t scalar(int32_t x) {
+    halide_scalar_value_t s;
+    s.u.i64 = 0;
+    s.u.i32 = x;
+    return s;
+}
+inline halide_scalar_value_t scalar(float x) {
+    halide_scalar_value_t s;
+    s.u.i64 = 0;
+    s.u.f32 = x;
+    return s;
+}
+
 }  // namespace hb
+
+// Exports F_argv and F_metadata for the extern "C" filter F, whose arguments ARGS describes in order.
+#define HB_EXPORT_FILTER(F, ARGS)                                                                          \
+    extern "C" int F##_argv(void **args) {                                                                 \
+        return hb::call_argv(F, args);                                                                     \
+    }                                                                                                      \
+    extern "C" const halide_filter_metadata_t *F##_metadata(void) {                                        \
+        static const halide_filter_metadata_t md = {1, (int32_t)(sizeof(ARGS) / sizeof(ARGS[0])), ARGS,    \
+                                                    hb::kTarget, #F};                                      \
+        return &md;                                                                                        \
+    }
+
+// The harnesses' second AOT variant F_auto_schedule: F itself under a second name, with its own argv and metadata.
+#define HB_EXPORT_AUTO_SCHEDULE(F, ARGS)                                          \
+    extern "C" decltype(F) F##_auto_schedule __attribute__((alias(#F)));         \
+    HB_EXPORT_FILTER(F##_auto_schedule, ARGS)
 
 // Launch macro: counts the launch, optionally brackets it with events for the per-kernel
 // profile (halide_b200_profile_*), and surfaces launch-configuration errors immediately.

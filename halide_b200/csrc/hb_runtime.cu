@@ -525,19 +525,19 @@ void *debug_fill(void *p, size_t bytes, cudaStream_t s) {
     return p;
 }
 
-static const char *kind(const ArgSpec &s) {
-    return s.is_output ? "Output" : "Input";
+static const char *kind(const halide_filter_argument_t &s) {
+    return s.kind == halide_argument_kind_output_buffer ? "Output" : "Input";
 }
 
-int check_arg(const halide_buffer_t *b, const ArgSpec &spec) {
+int check_arg(const halide_buffer_t *b, const halide_filter_argument_t &spec) {
     if (!b) {
         return fail(halide_error_code_buffer_argument_is_null, "Buffer argument %s is nullptr", spec.name);
     }
     // Compare code+bits only: this reference keeps the upper 16 bits reserved=0 while Halide
     // releases store lanes=1 there (SURVEY.md §8b "Type word").
-    if (b->type.code != spec.code || b->type.bits != spec.bits) {
+    if (b->type.code != spec.type.code || b->type.bits != spec.type.bits) {
         return fail(halide_error_code_bad_type, "%s buffer %s has type code %d bits %d but expected code %d bits %d",
-                    kind(spec), spec.name, b->type.code, b->type.bits, spec.code, spec.bits);
+                    kind(spec), spec.name, b->type.code, b->type.bits, spec.type.code, spec.type.bits);
     }
     if (b->dimensions != spec.dimensions) {
         return fail(halide_error_code_bad_dimensions, "%s buffer %s requires a buffer of exactly %d dimensions, but the buffer passed in has %d dimensions",
@@ -549,7 +549,7 @@ int check_arg(const halide_buffer_t *b, const ArgSpec &spec) {
     return 0;
 }
 
-int check_shape(const halide_buffer_t *b, const ArgSpec &spec) {
+int check_shape(const halide_buffer_t *b, const halide_filter_argument_t &spec) {
     int64_t total = 1;
     for (int d = 0; d < b->dimensions; d++) {
         const halide_dimension_t &dm = b->dim[d];
@@ -578,7 +578,7 @@ int check_shape(const halide_buffer_t *b, const ArgSpec &spec) {
     return 0;
 }
 
-int check_covers(const halide_buffer_t *b, const ArgSpec &spec, int d, int req_min, int req_extent) {
+int check_covers(const halide_buffer_t *b, const halide_filter_argument_t &spec, int d, int req_min, int req_extent) {
     if (req_extent <= 0) return 0;
     const halide_dimension_t &dm = b->dim[d];
     int req_max = req_min + req_extent - 1;
@@ -603,7 +603,7 @@ void propose_shape(halide_buffer_t *b, const int *mins, const int *extents) {
     }
 }
 
-int acquire_input(halide_buffer_t *b, const ArgSpec &spec, void **dev_ptr) {
+int acquire_input(halide_buffer_t *b, const halide_filter_argument_t &spec, void **dev_ptr) {
     if (b->device && b->device_interface != &g_cuda_interface) {
         return fail(halide_error_code_incompatible_device_interface,
                     "Input buffer %s has a device allocation of a different device interface", spec.name);
@@ -617,7 +617,7 @@ int acquire_input(halide_buffer_t *b, const ArgSpec &spec, void **dev_ptr) {
     return 0;
 }
 
-int acquire_output(halide_buffer_t *b, const ArgSpec &spec, void **dev_ptr) {
+int acquire_output(halide_buffer_t *b, const halide_filter_argument_t &spec, void **dev_ptr) {
     if (b->device && b->device_interface != &g_cuda_interface) {
         return fail(halide_error_code_incompatible_device_interface,
                     "Output buffer %s has a device allocation of a different device interface", spec.name);
@@ -788,7 +788,7 @@ uint64_t halide_b200_kernel_launch_count(void) {
     return g_launches.load();
 }
 const char *halide_b200_target(void) {
-    return "x86-64-linux-cuda-cuda_capability_100-b200_native";
+    return hb::kTarget;
 }
 
 void halide_b200_debug_fill_allocations(int byte) {

@@ -20,6 +20,8 @@
 #include <mutex>
 #include <vector>
 
+#include "../../include/local_laplacian.h"
+#include "../../include/local_laplacian_auto_schedule.h"
 #include "hb_dist.h"
 #include "ll_kernels.cuh"
 
@@ -30,30 +32,17 @@ using namespace llk;
 int g_shard_coarse_level = 0;  // halide_b200_ll_shard_coarse_level: 0 = choose by size, n >= 2 = gather level n
 int g_force_naive = 0;  // test hook bitmask (halide_b200_ll_force_generic): 1 = generic down kernels, 2 = generic up, 4 = generic final, 8 = no fused coarse launch, 16 = general-layout final kernel, 64 = no TMA frame tile in the final kernel, 256 = 48-row tiles in the TMA final kernel (default 32; 128 = 32 rows explicitly)
 
-const hb::ArgSpec kIn = {"input", halide_type_uint, 16, 3, false};
-const hb::ArgSpec kOut = {"output", halide_type_uint, 16, 3, true};
-
-int64_t est_i[3][2] = {{0, 1536}, {0, 2560}, {0, 3}};
-const int64_t *const est_ptrs[6] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1], &est_i[2][0], &est_i[2][1]};
-halide_scalar_value_t sv_levels, sv_alpha, sv_beta;
-struct InitScalars {
-    InitScalars() {
-        sv_levels.u.i64 = 0; sv_levels.u.i32 = 8;
-        sv_alpha.u.i64 = 0; sv_alpha.u.f32 = 1.0f;
-        sv_beta.u.i64 = 0; sv_beta.u.f32 = 1.0f;
-    }
-} init_scalars;
+const hb::BufferEstimates est({0, 1536, 0, 2560, 0, 3});
+const halide_scalar_value_t sv_levels = hb::scalar(8), sv_alpha = hb::scalar(1.0f), sv_beta = hb::scalar(1.0f);
 // Argument records as the generator declares them (generator :12-16, estimates :92-99).
 const halide_filter_argument_t kArgs[5] = {
-    {"input", halide_argument_kind_input_buffer, 3, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"input", halide_argument_kind_input_buffer, 3, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
     {"levels", halide_argument_kind_input_scalar, 0, {halide_type_int, 32, 0}, nullptr, nullptr, nullptr, &sv_levels, nullptr},
     {"alpha", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv_alpha, nullptr},
     {"beta", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv_beta, nullptr},
-    {"output", halide_argument_kind_output_buffer, 3, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"output", halide_argument_kind_output_buffer, 3, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
 };
-const halide_filter_metadata_t kMeta = {1, 5, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "local_laplacian"};
-const halide_filter_metadata_t kMetaAuto = {1, 5, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "local_laplacian_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[4];
 
 
 // Everything one call needs on the device: frame description + per-level buffers.
@@ -405,35 +394,6 @@ void run_coarse_sweep(Plan &p, int from_level, cudaStream_t s) {
     for (int j = j0; j > from_level; j--) launch_up(p, j, s);
 }
 
-int run_local_laplacian(halide_buffer_t *input, int levels, float alpha, float beta, halide_buffer_t *output) {
-    int r;
-    bool done;
-    if ((r = check_and_query(input, levels, output, &done)) || done) return r;
-    void *din = nullptr, *dout = nullptr;
-    if ((r = hb::acquire_input(input, kIn, &din))) return r;
-    if ((r = hb::acquire_output(output, kOut, &dout))) return r;
-
-    Plan p;
-    fill_frame(p, input, output, din, dout, levels, alpha, beta);
-    const int W = p.f.W, H = p.f.H;
-    Span outx = {p.f.out_x0, p.f.out_x0 + W - 1}, outy = {p.f.out_y0, p.f.out_y0 + H - 1};
-    Span inx = {p.f.in_x0, p.f.in_x0 + p.f.in_w - 1}, iny = {p.f.in_y0, p.f.in_y0 + p.f.in_h - 1};
-    p.geom = ll::make_geom(outx, outy, inx, iny, p.J);
-    hb::Scratch scratch;
-    if ((r = alloc_levels(p, scratch))) return r;
-
-    cudaStream_t s = hb::stream();
-    if ((r = get_lut(p, s))) return r;
-    {
-        hb::CallTimer timer(s);
-        run_coarse_sweep(p, 0, s);
-        launch_final(p, s);
-    }
-    if ((r = hb::check_cuda(cudaGetLastError(), "local_laplacian launch", halide_error_code_device_run_failed))) return r;
-    hb::mark_output_written(output);
-    return 0;
-}
-
 // Row-sharded path: the level gathered all-to-all (levels from it upwards are replicated on every rank).
 // Depends only on the whole frame's geometry and the rank count, so every rank computes the same value.
 int choose_coarse_level(const ll::Geom &whole, int nranks, int J, int K) {
@@ -700,26 +660,37 @@ int run_local_laplacian_sharded(halide_buffer_t *input, int levels, float alpha,
 }  // namespace
 
 extern "C" int local_laplacian(halide_buffer_t *input, int32_t levels, float alpha, float beta, halide_buffer_t *output) {
-    return run_local_laplacian(input, levels, alpha, beta, output);
+    int r;
+    bool done;
+    if ((r = check_and_query(input, levels, output, &done)) || done) return r;
+    void *din = nullptr, *dout = nullptr;
+    if ((r = hb::acquire_input(input, kIn, &din))) return r;
+    if ((r = hb::acquire_output(output, kOut, &dout))) return r;
+
+    Plan p;
+    fill_frame(p, input, output, din, dout, levels, alpha, beta);
+    const int W = p.f.W, H = p.f.H;
+    Span outx = {p.f.out_x0, p.f.out_x0 + W - 1}, outy = {p.f.out_y0, p.f.out_y0 + H - 1};
+    Span inx = {p.f.in_x0, p.f.in_x0 + p.f.in_w - 1}, iny = {p.f.in_y0, p.f.in_y0 + p.f.in_h - 1};
+    p.geom = ll::make_geom(outx, outy, inx, iny, p.J);
+    hb::Scratch scratch;
+    if ((r = alloc_levels(p, scratch))) return r;
+
+    cudaStream_t s = hb::stream();
+    if ((r = get_lut(p, s))) return r;
+    {
+        hb::CallTimer timer(s);
+        run_coarse_sweep(p, 0, s);
+        launch_final(p, s);
+    }
+    if ((r = hb::check_cuda(cudaGetLastError(), "local_laplacian launch", halide_error_code_device_run_failed))) return r;
+    hb::mark_output_written(output);
+    return 0;
 }
-extern "C" int local_laplacian_argv(void **args) {
-    return run_local_laplacian((halide_buffer_t *)args[0], *(int32_t *)args[1], *(float *)args[2], *(float *)args[3],
-                               (halide_buffer_t *)args[4]);
-}
-extern "C" const halide_filter_metadata_t *local_laplacian_metadata(void) {
-    return &kMeta;
-}
+
+HB_EXPORT_FILTER(local_laplacian, kArgs)
 // The harness's second AOT variant (apps/local_laplacian/process.cpp:44-48): same implementation.
-extern "C" int local_laplacian_auto_schedule(halide_buffer_t *input, int32_t levels, float alpha, float beta,
-                                             halide_buffer_t *output) {
-    return run_local_laplacian(input, levels, alpha, beta, output);
-}
-extern "C" int local_laplacian_auto_schedule_argv(void **args) {
-    return local_laplacian_argv(args);
-}
-extern "C" const halide_filter_metadata_t *local_laplacian_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_AUTO_SCHEDULE(local_laplacian, kArgs)
 
 // Test hook: route K == 8 calls through the generic (any `levels`) kernels so both paths stay covered.
 extern "C" void halide_b200_ll_force_generic(int enable) {

@@ -14,6 +14,8 @@
 //   A  d for all dx over the tile grown by the patch apron          -> smem D[dx][y][x]
 //   B  vertical patch sums                                          -> smem V[dx][y][x]
 //   C  horizontal patch sums, fast_exp, accumulate 4 running sums in registers (2 px per thread)
+#include "../../include/nl_means.h"
+#include "../../include/nl_means_auto_schedule.h"
 #include "hb_common.h"
 #include "hl_math.cuh"
 
@@ -210,30 +212,24 @@ constexpr size_t nl_window_smem() {
 constexpr bool kDefaultWindow = true;  // (the register-window kernel: bit-identical to the first kernel on hardware, profiles/r02_ab_variants.log)
 int g_variant = 0;  // test / A-B hook (halide_b200_nl_means_variant): 0 = default, 1 = generic kernel, 2 = register-window kernel
 
-const hb::ArgSpec kIn = {"input", halide_type_float, 32, 3, false};
-const hb::ArgSpec kOut = {"non_local_means", halide_type_float, 32, 3, true};
-int64_t est_i[3][2] = {{0, 1536}, {0, 2560}, {0, 3}};
-const int64_t *const est_ptrs[6] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1], &est_i[2][0], &est_i[2][1]};
-halide_scalar_value_t sv_patch, sv_search, sv_sigma;
-struct InitScalars {
-    InitScalars() {
-        sv_patch.u.i64 = 0; sv_patch.u.i32 = 7;
-        sv_search.u.i64 = 0; sv_search.u.i32 = 7;
-        sv_sigma.u.i64 = 0; sv_sigma.u.f32 = 0.12f;
-    }
-} init_scalars;
+const hb::BufferEstimates est({0, 1536, 0, 2560, 0, 3});
+const halide_scalar_value_t sv_patch = hb::scalar(7), sv_search = hb::scalar(7), sv_sigma = hb::scalar(0.12f);
 const halide_filter_argument_t kArgs[5] = {
-    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
     {"patch_size", halide_argument_kind_input_scalar, 0, {halide_type_int, 32, 0}, nullptr, nullptr, nullptr, &sv_patch, nullptr},
     {"search_area", halide_argument_kind_input_scalar, 0, {halide_type_int, 32, 0}, nullptr, nullptr, nullptr, &sv_search, nullptr},
     {"sigma", halide_argument_kind_input_scalar, 0, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, &sv_sigma, nullptr},
-    {"non_local_means", halide_argument_kind_output_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"non_local_means", halide_argument_kind_output_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
 };
-const halide_filter_metadata_t kMeta = {1, 5, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "nl_means"};
-const halide_filter_metadata_t kMetaAuto = {1, 5, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "nl_means_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[4];
 
-int run_nl_means(halide_buffer_t *input, int patch_size, int search_area, float sigma, halide_buffer_t *output) {
+}  // namespace
+
+extern "C" void halide_b200_nl_means_variant(int v) {
+    g_variant = v;
+}
+
+extern "C" int nl_means(halide_buffer_t *input, int32_t patch_size, int32_t search_area, float sigma, halide_buffer_t *output) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(output, kOut))) return r;
@@ -316,29 +312,5 @@ int run_nl_means(halide_buffer_t *input, int patch_size, int search_area, float 
     return 0;
 }
 
-}  // namespace
-
-extern "C" void halide_b200_nl_means_variant(int v) {
-    g_variant = v;
-}
-
-extern "C" int nl_means(halide_buffer_t *input, int32_t patch_size, int32_t search_area, float sigma, halide_buffer_t *output) {
-    return run_nl_means(input, patch_size, search_area, sigma, output);
-}
-extern "C" int nl_means_argv(void **args) {
-    return run_nl_means((halide_buffer_t *)args[0], *(int32_t *)args[1], *(int32_t *)args[2], *(float *)args[3],
-                        (halide_buffer_t *)args[4]);
-}
-extern "C" const halide_filter_metadata_t *nl_means_metadata(void) {
-    return &kMeta;
-}
-extern "C" int nl_means_auto_schedule(halide_buffer_t *input, int32_t patch_size, int32_t search_area, float sigma,
-                                      halide_buffer_t *output) {
-    return run_nl_means(input, patch_size, search_area, sigma, output);
-}
-extern "C" int nl_means_auto_schedule_argv(void **args) {
-    return nl_means_argv(args);
-}
-extern "C" const halide_filter_metadata_t *nl_means_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(nl_means, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(nl_means, kArgs)

@@ -15,6 +15,8 @@
 // compulsory HBM traffic).  kFuse stages run per launch on a shared-memory tile with a 2*kFuse
 // apron, ping-ponging between two uint16 tiles; the frame itself (7.9 MB at the harness size)
 // stays L2-resident between launches.
+#include "../../include/stencil_chain.h"
+#include "../../include/stencil_chain_auto_schedule.h"
 #include "hb_common.h"
 
 namespace {
@@ -227,19 +229,20 @@ __global__ void __launch_bounds__(256) stencil_chain_window_kernel(Plane p) {
 constexpr bool kDefaultWindow = true;  // (the register-window kernel: bit-identical to the first kernel on hardware, profiles/r02_ab_variants.log)
 int g_variant = 0;  // test / A-B hook (halide_b200_stencil_chain_variant): 0 = default, 1 = one-pixel-per-thread kernel, 2 = register-window kernel
 
-const hb::ArgSpec kIn = {"input", halide_type_uint, 16, 2, false};
-const hb::ArgSpec kOut = {"output", halide_type_uint, 16, 2, true};
-int64_t est_i[2][2] = {{0, 1536}, {0, 2560}};
-const int64_t *const est_ptrs[4] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1]};
+const hb::BufferEstimates est({0, 1536, 0, 2560});
 const halide_filter_argument_t kArgs[2] = {
-    {"input", halide_argument_kind_input_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
-    {"output", halide_argument_kind_output_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"input", halide_argument_kind_input_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
+    {"output", halide_argument_kind_output_buffer, 2, {halide_type_uint, 16, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
 };
-const halide_filter_metadata_t kMeta = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "stencil_chain"};
-const halide_filter_metadata_t kMetaAuto = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "stencil_chain_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[1];
 
-int run_stencil_chain(halide_buffer_t *input, halide_buffer_t *output) {
+}  // namespace
+
+extern "C" void halide_b200_stencil_chain_variant(int v) {
+    g_variant = v;
+}
+
+extern "C" int stencil_chain(halide_buffer_t *input, halide_buffer_t *output) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(output, kOut))) return r;
@@ -328,27 +331,5 @@ int run_stencil_chain(halide_buffer_t *input, halide_buffer_t *output) {
     return 0;
 }
 
-}  // namespace
-
-extern "C" void halide_b200_stencil_chain_variant(int v) {
-    g_variant = v;
-}
-
-extern "C" int stencil_chain(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_stencil_chain(input, output);
-}
-extern "C" int stencil_chain_argv(void **args) {
-    return run_stencil_chain((halide_buffer_t *)args[0], (halide_buffer_t *)args[1]);
-}
-extern "C" const halide_filter_metadata_t *stencil_chain_metadata(void) {
-    return &kMeta;
-}
-extern "C" int stencil_chain_auto_schedule(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_stencil_chain(input, output);
-}
-extern "C" int stencil_chain_auto_schedule_argv(void **args) {
-    return stencil_chain_argv(args);
-}
-extern "C" const halide_filter_metadata_t *stencil_chain_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(stencil_chain, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(stencil_chain, kArgs)

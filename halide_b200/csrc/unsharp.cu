@@ -16,6 +16,8 @@
 // multiply reads the staged centre pixels.  Algorithmic traffic is 24 B/px (12 in, 12 out) against ~60 flops/px.
 #include <math.h>
 
+#include "../../include/unsharp.h"
+#include "../../include/unsharp_auto_schedule.h"
 #include "hb_common.h"
 #include "hb_tile.cuh"
 
@@ -111,19 +113,16 @@ __global__ void __launch_bounds__(NT) unsharp_kernel(UnsharpParams q) {
     }
 }
 
-const hb::ArgSpec kIn = {"input", halide_type_float, 32, 3, false};
-const hb::ArgSpec kOut = {"output", halide_type_float, 32, 3, true};
-int64_t est_i[3][2] = {{0, 1536}, {0, 2560}, {0, 3}};
-const int64_t *const est_ptrs[6] = {&est_i[0][0], &est_i[0][1], &est_i[1][0], &est_i[1][1], &est_i[2][0], &est_i[2][1]};
+const hb::BufferEstimates est({0, 1536, 0, 2560, 0, 3});
 const halide_filter_argument_t kArgs[2] = {
-    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
-    {"output", halide_argument_kind_output_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est_ptrs},
+    {"input", halide_argument_kind_input_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
+    {"output", halide_argument_kind_output_buffer, 3, {halide_type_float, 32, 0}, nullptr, nullptr, nullptr, nullptr, est.p},
 };
-const halide_filter_metadata_t kMeta = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native", "unsharp"};
-const halide_filter_metadata_t kMetaAuto = {1, 2, kArgs, "x86-64-linux-cuda-cuda_capability_100-b200_native",
-                                            "unsharp_auto_schedule"};
+const auto &kIn = kArgs[0], &kOut = kArgs[1];
 
-int run_unsharp(halide_buffer_t *input, halide_buffer_t *output) {
+}  // namespace
+
+extern "C" int unsharp(halide_buffer_t *input, halide_buffer_t *output) {
     int r;
     if ((r = hb::check_arg(input, kIn))) return r;
     if ((r = hb::check_arg(output, kOut))) return r;
@@ -168,23 +167,5 @@ int run_unsharp(halide_buffer_t *input, halide_buffer_t *output) {
     return 0;
 }
 
-}  // namespace
-
-extern "C" int unsharp(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_unsharp(input, output);
-}
-extern "C" int unsharp_argv(void **args) {
-    return run_unsharp((halide_buffer_t *)args[0], (halide_buffer_t *)args[1]);
-}
-extern "C" const halide_filter_metadata_t *unsharp_metadata(void) {
-    return &kMeta;
-}
-extern "C" int unsharp_auto_schedule(halide_buffer_t *input, halide_buffer_t *output) {
-    return run_unsharp(input, output);
-}
-extern "C" int unsharp_auto_schedule_argv(void **args) {
-    return unsharp_argv(args);
-}
-extern "C" const halide_filter_metadata_t *unsharp_auto_schedule_metadata(void) {
-    return &kMetaAuto;
-}
+HB_EXPORT_FILTER(unsharp, kArgs)
+HB_EXPORT_AUTO_SCHEDULE(unsharp, kArgs)

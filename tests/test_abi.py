@@ -1,13 +1,31 @@
 """CPU tests of the drop-in boundary: the library loads and exports every symbol include/*.h
-declares; struct layouts match the LP64 facts of src/runtime/HalideRuntime.h:1657-1737."""
+declares; struct layouts match the LP64 facts of src/runtime/HalideRuntime.h:1657-1737; every F_metadata() record
+matches the committed snapshot; every F_argv unpacks its arguments as F declares them."""
 import ctypes
 import glob
+import importlib.util
+import json
 import os
 import re
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+
+def _load_metadata_dumper():
+    spec = importlib.util.spec_from_file_location("make_abi_metadata", os.path.join(GOLDEN, "make_abi_metadata.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+META = _load_metadata_dumper()
+with open(os.path.join(GOLDEN, "abi_metadata.json")) as _f:
+    SNAPSHOT = json.load(_f)
+FILTERS = sorted(SNAPSHOT)
 
 
 def _declared_symbols():
@@ -16,11 +34,8 @@ def _declared_symbols():
         text = open(h).read()
         text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
         text = re.sub(r"//[^\n]*", "", text)
-        for m in re.finditer(r"^[A-Za-z_][\w \*]*?\b(\w+)\s*\([^;{]*\)\s*;", text, flags=re.M):
-            name = m.group(1)
-            if name.startswith(("halide_", "local_laplacian", "bilateral_grid", "nl_means", "stencil_chain",
-                                "conv_layer", "camera_pipe")):
-                syms.add(name)
+        for m in re.finditer(r"^(?!typedef\b)[A-Za-z_][\w \*]*?\b(\w+)\s*\([^;{]*\)\s*;", text, flags=re.M):
+            syms.add(m.group(1))
     return sorted(syms)
 
 
@@ -42,17 +57,54 @@ def test_struct_layout(hb):
 
 
 def test_metadata_and_target(hb):
+    """tests/golden/abi_metadata.json holds one record per filter header, and every filter reports the library's own
+    target string."""
     l = hb.load_library()
+    assert FILTERS == META.filter_functions()
+    target = hb.capi.halide_b200_target().decode()
+    assert target.endswith("b200_native")
+    assert [META.dump(l, fn)["target"] for fn in FILTERS] == [target] * len(FILTERS)
 
-    class Meta(ctypes.Structure):
-        _fields_ = [("version", ctypes.c_int32), ("num_arguments", ctypes.c_int32), ("arguments", ctypes.c_void_p),
-                    ("target", ctypes.c_char_p), ("name", ctypes.c_char_p)]
-    l.local_laplacian_metadata.restype = ctypes.POINTER(Meta)
-    md = l.local_laplacian_metadata().contents
-    assert md.version == 1 and md.num_arguments == 5 and md.name == b"local_laplacian"
-    assert b"cuda" in md.target
-    l.halide_blur_metadata.restype = ctypes.POINTER(Meta)
-    assert l.halide_blur_metadata().contents.num_arguments == 2
+
+@pytest.mark.parametrize("fn", FILTERS)
+def test_metadata_matches_snapshot(hb, fn):
+    """The library reports each F_metadata() record of the snapshot field for field: names, kinds, types, scalar and
+    buffer estimates, target and name."""
+    assert META.dump(hb.load_library(), fn) == SNAPSHOT[fn]
+
+
+_DTYPES = {(0, 32): np.int32, (1, 8): np.uint8, (1, 16): np.uint16, (2, 32): np.float32}
+
+
+@pytest.mark.parametrize("fn", FILTERS)
+def test_argv_matches_direct_call(hb, fn):
+    """F_argv(args) is F called with *args[i] for scalars and args[i] for buffers (src/CodeGen_C.cpp:675-705).  Every
+    buffer is a bounds query, which F answers before any CUDA call: both calls must return 0 and propose the same
+    shapes.  Each buffer starts from its metadata estimates shifted by its position, so a swapped pair shows."""
+    from halide_b200 import HalideBuffer
+    from halide_b200.buffer import halide_buffer_t
+    l = hb.load_library()
+    args = SNAPSHOT[fn]["arguments"]
+
+    def call(via_argv):
+        bufs, values = [], []
+        for i, a in enumerate(args):
+            if a["kind"] == 0:
+                values.append((ctypes.c_int32 if a["type"][0] == 0 else ctypes.c_float)(a["scalar_estimate"]))
+            else:
+                est = a["buffer_estimates"] or [0, 64] * a["dimensions"]
+                b = HalideBuffer(_DTYPES[tuple(a["type"][:2])], est[1::2], mins=[m + i for m in est[0::2]])
+                bufs.append(b)
+                values.append(b.buf)
+        if via_argv:
+            argv = (ctypes.c_void_p * len(values))(*[ctypes.addressof(v) for v in values])
+            rc = getattr(l, fn + "_argv")(argv)
+        else:
+            rc = getattr(l, fn)(*[ctypes.byref(v) if isinstance(v, halide_buffer_t) else v for v in values])
+        return rc, [b.shape() for b in bufs]
+
+    direct, via_argv = call(False), call(True)
+    assert direct[0] == 0 and via_argv == direct
 
 
 def test_validation_errors_without_gpu(hb):

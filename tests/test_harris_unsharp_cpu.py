@@ -1,9 +1,8 @@
 """CPU tests of harris and unsharp: the oracle against the committed golden vectors and against the independent numpy
 restatement (oracle/np_restatement_apps.py), the folded unsharp weights, and the C-ABI entry points up to the first
-CUDA call (export, metadata, validation error codes, bounds queries, a C caller that links)."""
-import ctypes
+CUDA call (validation error codes, bounds queries); tests/test_abi.py and tests/test_headers_compile.py check their
+export, metadata and _argv with every other filter's."""
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -12,10 +11,6 @@ from util import f32_frame
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-INC = os.path.join(ROOT, "include")
-LIBDIR = os.path.join(ROOT, "halide_b200")
-ENTRY_POINTS = [f + s for f in ("harris", "unsharp") for s in ("", "_argv", "_metadata", "_auto_schedule", "_auto_schedule_argv",
-                                                              "_auto_schedule_metadata")]
 
 
 @pytest.fixture(scope="module")
@@ -145,40 +140,6 @@ def test_unsharp_oracle_rejects_non_covering_inputs(apps):
 
 # ---- the C ABI without a GPU ---------------------------------------------------------------------------------------------
 
-class Arg(ctypes.Structure):
-    _fields_ = [("name", ctypes.c_char_p), ("kind", ctypes.c_int32), ("dimensions", ctypes.c_int32), ("type", ctypes.c_uint32),
-                ("scalar", ctypes.c_void_p * 4), ("buffer_estimates", ctypes.POINTER(ctypes.POINTER(ctypes.c_int64)))]
-
-
-class Meta(ctypes.Structure):
-    _fields_ = [("version", ctypes.c_int32), ("num_arguments", ctypes.c_int32), ("arguments", ctypes.POINTER(Arg)),
-                ("target", ctypes.c_char_p), ("name", ctypes.c_char_p)]
-
-
-def test_entry_points_exported(hb):
-    l = hb.load_library()
-    assert [s for s in ENTRY_POINTS if not hasattr(l, s)] == []
-
-
-@pytest.mark.parametrize("name,estimates", [
-    ("harris", [[0, 1536, 0, 2560, 0, 3], [3, 1530, 3, 2554]]),
-    ("unsharp", [[0, 1536, 0, 2560, 0, 3], [0, 1536, 0, 2560, 0, 3]]),
-])
-def test_metadata(hb, name, estimates):
-    l = hb.load_library()
-    for suffix in ("", "_auto_schedule"):
-        fn = getattr(l, name + suffix + "_metadata")
-        fn.restype = ctypes.POINTER(Meta)
-        md = fn().contents
-        assert md.version == 1 and md.num_arguments == 2 and md.name == (name + suffix).encode()
-        assert b"cuda" in md.target
-        for i, (want_name, kind, est) in enumerate(zip((b"input", b"output"), (1, 2), estimates)):
-            a = md.arguments[i]
-            assert a.name == want_name and a.kind == kind and a.dimensions == len(est) // 2
-            assert a.type & 0xFFFF == (32 << 8) | 2  # float32
-            assert [a.buffer_estimates[k][0] for k in range(len(est))] == est
-
-
 def _expect(code, fn, *args):
     from halide_b200 import HalideError
     with pytest.raises(HalideError) as e:
@@ -246,24 +207,3 @@ def test_bounds_queries(hb):
     q = B.bounds_query(np.float32, 3)
     assert F.unsharp(q, B.from_numpy(np.zeros((4, 20, 30), np.float32), mins=(-3, 5, 1))) == 0
     assert q.shape() == [(-3, 30, 1), (5, 20, 30), (1, 4, 600)]
-
-
-def test_c_caller_links_the_new_entry_points(tmp_path):
-    if not os.path.exists(os.path.join(LIBDIR, "libhalide_b200.so")):
-        pytest.skip("library not built")
-    body = '#include "halide_b200_runtime.h"\n'
-    body += "".join(f'#include "{n}{s}.h"\n' for n in ("harris", "unsharp") for s in ("", "_auto_schedule"))
-    body += "#include <stdio.h>\nint main(void) {\n  const struct halide_filter_metadata_t *m;\n"
-    for n in ("harris", "unsharp", "harris_auto_schedule", "unsharp_auto_schedule"):
-        body += f'  m = {n}_metadata();\n  if (!m || !m->name) return 1;\n  printf("%s %d\\n", m->name, m->num_arguments);\n'
-        body += f"  {{ int (*fp)(void **) = {n}_argv; if (!fp) return 2; }}\n"
-        body += f"  {{ int (*fp)(struct halide_buffer_t *, struct halide_buffer_t *) = {n}; if (!fp) return 3; }}\n"
-    body += "  return 0;\n}\n"
-    src, exe = tmp_path / "caller.c", tmp_path / "caller"
-    src.write_text(body)
-    out = subprocess.run(["/usr/bin/gcc", "-std=c99", "-Wall", "-Werror", f"-I{INC}", str(src), "-o", str(exe), f"-L{LIBDIR}",
-                          "-lhalide_b200", f"-Wl,-rpath,{LIBDIR}", "-lpthread", "-ldl"], capture_output=True, text=True, timeout=120)
-    assert out.returncode == 0, out.stderr[-2000:]
-    run = subprocess.run([str(exe)], capture_output=True, text=True, timeout=60)  # metadata only: no CUDA call
-    assert run.returncode == 0, run.stdout + run.stderr
-    assert run.stdout.split("\n")[:4] == ["harris 2", "unsharp 2", "harris_auto_schedule 2", "unsharp_auto_schedule 2"]
